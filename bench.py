@@ -19,6 +19,10 @@ ranks; each region is repeated ``--repeats`` times (K steps each) and the MEDIAN
 * ``e2e``    — the same K steps through the public API (``model.train_iter`` + ``exchanger.exchange``): every step the
   loader copies a fresh uint8 batch from pinned host memory (H2D) and the host reads the step's loss back (D2H).
 
+The device-resident batch of the ``value`` region is drawn from a fixed seed, so runs with the same arguments see the same
+inputs; ``--dump-outputs DIR`` writes what the last step of that region returned, and the weights it left, as ``DIR/*.npy``
+so that two builds can be compared output for output.
+
 ``--impl reference`` runs the unmodified reference from ``baseline/_ref`` if it can run (it cannot in this image: Theano /
 pygpu / mpi4py / mpirun are not installable offline).  ``--impl torch_best`` is the strongest same-semantics LIBRARY build
 (cuDNN / cuBLAS channels-last, CUDA-graph-captured step, fused foreach momentum-SGD, one flat-bucket ncclAllReduce);
@@ -53,6 +57,8 @@ MODELS = {
     "resnet50": ("theanompi_b200.models.lasagne_model_zoo.resnet50", "ResNet50", dict(batch_size=64, file_batch_size=64), "3x224x224"),
     "wrn": ("theanompi_b200.models.keras_model_zoo.wresnet", "Wide_ResNet", dict(batch_size=128, file_batch_size=128), "3x32x32"),
 }
+INPUT_SEED = 1234          # the device-resident batch of the timed region: the same pixels and labels on every run
+DUMP_WEIGHTS = 1 << 22     # --dump-outputs: weights sampled beyond this many values (16 MiB of float32)
 
 
 def parse():
@@ -71,7 +77,14 @@ def parse():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-overlap", action="store_true")
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch (default: the published one for the model)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step of the device-timed region returned (cost.npy, error.npy) "
+                         "and the weights it left (weights.npy: all of them, or a fixed seeded sample of %d) as float32 .npy files "
+                         "(BSP rule, --impl ours)" % DUMP_WEIGHTS)
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.rule != "bsp"):
+        ap.error("--dump-outputs needs --impl ours --rule bsp")
+    return args
 
 
 class ClockSampler(object):
@@ -204,11 +217,33 @@ def model_cfg(args, name, world_for_data):
 
 
 def set_device_batch(model, torch, dev):
-    """Device-resident batch for the kernel-timed region (random pixels of the model's input shape, random labels)."""
+    """Device-resident batch for the kernel-timed region (seeded random pixels of the model's input shape, random labels)."""
     shp = tuple(model.shared_x.shape)
-    model.shared_x = torch.randn(shp, device=dev).to(model.act_dtype)
+    g = torch.Generator(device=dev)
+    g.manual_seed(INPUT_SEED)
+    model.shared_x = torch.randn(shp, device=dev, generator=g).to(model.act_dtype)
     hi = int(getattr(model, "n_softmax_out", 0) or getattr(model.data, "n_class", 10))
-    model.shared_y.copy_(torch.randint(0, hi, (shp[0],), device=dev))
+    model.shared_y.copy_(torch.randint(0, hi, (shp[0],), device=dev, generator=g))
+
+
+def step_outputs(model, out, torch):
+    """Host copies of what a training step hands back: its (cost, error) and the model's weights after the update — all of
+    them, or a fixed seeded sample of DUMP_WEIGHTS values taken in parameter order."""
+    import numpy as np
+    cost, error = out[:2]
+    w = torch.cat([p.detach().reshape(-1).float() for p in model.params])
+    if w.numel() > DUMP_WEIGHTS:
+        idx = np.sort(np.random.default_rng(0).choice(w.numel(), DUMP_WEIGHTS, replace=False))
+        w = w[torch.from_numpy(idx).to(w.device)]
+    return {"cost": cost.detach().float().reshape(1).cpu().numpy(), "error": error.detach().float().reshape(1).cpu().numpy(),
+            "weights": w.cpu().numpy()}
+
+
+def dump_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def e2e_loop(model, rec, step_extra, K, Wm, torch, start_count):
@@ -296,7 +331,11 @@ def run_bsp(args, rank, world, local):
     T.barrier()
     sampler = ClockSampler(local)
     sampler.start()
-    dev_ms = [T.region(dev_step, K)[0] for _ in range(R)]
+    dev_ms = []
+    for _ in range(R):
+        ms, last = T.region(dev_step, K)
+        dev_ms.append(ms)
+    outputs = step_outputs(model, last, torch) if args.dump_outputs else None
 
     # ---------------- end-to-end region through the public API (loader H2D + loss D2H every step)
     model.reset_iter("train")
@@ -319,6 +358,8 @@ def run_bsp(args, rank, world, local):
     if rank == 0:
         emit(args, world, K, Wm, stats(dev_ms, K), stats(e2e_ms, K), None, args.model, inp, batch, world, launches, h2d,
              losses[-1] if losses else None, clocks, "bsp", strategy if world > 1 else "local fused SGD")
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     model.cleanup()
     worker.finalize()
     return 0

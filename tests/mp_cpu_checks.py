@@ -1,6 +1,6 @@
 """Multi-process CPU (gloo) checks, launched by tests/test_distributed_cpu.py with RANK/WORLD_SIZE set.
 
-    python tests/mp_cpu_checks.py <case>
+    python tests/mp_cpu_checks.py <case> [case arguments]
 """
 import os
 import sys
@@ -96,16 +96,17 @@ def _tiny_model(p, sync_type, strategy, n_steps=6, lr=0.02):
     return m
 
 
-def case_bsp_equivalence():
+def case_bsp_equivalence(out_dir):
     """2 ranks × batch 16 with cdd exchange ≡ 1 process × batch 32 (the reference's
-    test-cdd-train idea with real asserts), for the host and 'nccl32'-semantics strategies."""
+    test-cdd-train idea with real asserts), for the host and 'nccl32'-semantics strategies.
+    Rank 0 writes the final weights of each strategy to ``out_dir/bsp_<strategy>.pt``."""
     p = _proc()
     for strat in ("ar", "nccl32", "asa32"):
         m = _tiny_model(p, "cdd", strat)
         ws = p.comm.allgather(m.arena.W.clone())
         assert torch.equal(ws[0], ws[1]), "replicas diverged (%s)" % strat
         if p.rank == 0:
-            torch.save(m.arena.W.clone(), "/tmp/tmpi_bsp_%s.pt" % strat)
+            torch.save(m.arena.W.clone(), os.path.join(out_dir, "bsp_%s.pt" % strat))
     p.comm.Barrier()
     print("OK bsp rank", p.rank)
 
@@ -119,7 +120,7 @@ def case_bsp_avg():
 
 
 if __name__ == "__main__":
-    globals()["case_" + sys.argv[1]]()
+    globals()["case_" + sys.argv[1]](*sys.argv[2:])
     if dist.is_initialized():
         dist.barrier()
         dist.destroy_process_group()

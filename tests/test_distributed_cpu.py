@@ -11,13 +11,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 _PORT = [29700]
 
 
-def run_ranks(n, case, timeout=240):
+def run_ranks(n, case, *args, timeout=240):
     _PORT[0] += 1
     procs = []
     for r in range(n):
         env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(n), LOCAL_RANK=str(r), MASTER_ADDR="127.0.0.1",
                    MASTER_PORT=str(_PORT[0]), OMP_NUM_THREADS="2", PYTHONPATH=ROOT)
-        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "mp_cpu_checks.py"), case], env=env,
+        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "mp_cpu_checks.py"), case] + list(args), env=env,
                                       stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
     outs = []
     for p in procs:
@@ -42,8 +42,8 @@ def test_mailbox_control_plane_world3():
     run_ranks(3, "mailbox")
 
 
-def test_bsp_cdd_two_ranks_equals_one_big_batch():
-    run_ranks(2, "bsp_equivalence")
+def test_bsp_cdd_two_ranks_equals_one_big_batch(tmp_path):
+    run_ranks(2, "bsp_equivalence", str(tmp_path))
     # single process, batch 32 = the two shards of each step concatenated
     from theanompi_b200.models import layers2
     from theanompi_b200.models.cifar10 import Cifar10_model
@@ -73,7 +73,7 @@ def test_bsp_cdd_two_ranks_equals_one_big_batch():
         m.sgd.step(m.shared_lr.get_value(), k=2)
     Dropout.SetDropoutOn(); Crop.SetRandCropOn()
     for strat in ("ar", "nccl32", "asa32"):
-        w2 = torch.load("/tmp/tmpi_bsp_%s.pt" % strat)
+        w2 = torch.load(str(tmp_path / ("bsp_%s.pt" % strat)))
         err = float((w2 - m.arena.W).abs().max())
         assert err < 2e-5, (strat, err)
 

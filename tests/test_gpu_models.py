@@ -162,7 +162,7 @@ def test_loader_process_mode_gpu(tmp_path, monkeypatch):
         ld.close()
 
 
-def test_deterministic_mode_is_bit_reproducible():
+def test_deterministic_mode_is_bit_reproducible(tmp_path):
     """TMPI_DETERMINISTIC=1 (no split-K: every gradient element is produced by one CTA in a fixed k order) → two runs of the same
     training steps give bit-identical weights; the default (split-K with fp32 atomics in arrival order) is only close."""
     import os
@@ -182,7 +182,7 @@ def test_deterministic_mode_is_bit_reproducible():
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     outs = []
     for k in range(2):
-        f = "/tmp/tmpi_det_%d.pt" % k
+        f = str(tmp_path / ("w%d.pt" % k))
         env = dict(os.environ, TMPI_DETERMINISTIC="1", PYTHONPATH=root)
         r = subprocess.run([sys.executable, "-c", code, f], env=env, cwd=root, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=300)
         assert r.returncode == 0, r.stdout[-2000:]
