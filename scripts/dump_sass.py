@@ -18,9 +18,10 @@ import sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SO = os.path.join(ROOT, "theanompi_b200", "_tmpi_native.so")
 OUT = os.path.join(ROOT, "profiles", "sass")
-FULL = ["gemm_tcgen05I13__nv_bfloat16Li128ELi2", "gemm_tcgen05IfLi128ELi1", "fused_twoshot_sgd_kernelILi8", "fused_oneshot_sgd_kernelILi4",
+FULL = ["gemm_tcgen05I13__nv_bfloat16Li128ELi2", "gemm_tcgen05IfLi128ELi1", "fused_twoshot_kernelINS_7SgdRuleELi8", "fused_oneshot_kernelINS_7SgdRuleELi4",
+        "fused_twoshot_kernelINS_8AdamRuleELi8", "fused_oneshot_kernelINS_8AdamRuleELi4",
         "easgd_elastic_kernelILi4", "gosgd_pull_merge_kernelILi4", "ticket_acquire_kernel", "ticket_release_kernel", "gosgd_poll_kernel",
-        "gosgd_push_end_kernel", "push_master_kernel", "sgd_flat_kernel", "adam_flat_kernel", "bn_colreduce_kernelI13__nv_bfloat16Li1",
+        "gosgd_push_end_kernel", "push_region_kernel", "sgd_flat_kernel", "adam_flat_kernel", "bn_colreduce_kernelI13__nv_bfloat16Li1",
         "bn_apply_kernelI13__nv_bfloat16", "lstm_cell_fwd_kernelI13__nv_bfloat16"]
 
 

@@ -34,7 +34,12 @@ struct FusedArgs {
   int push_master = 1;                               // two-shot: 1 = push the updated fp32 master slice AND the bf16 shadow to every peer;
                                                      // 0 = owner keeps the master of WEIGHT blocks (group 0): peers receive only their bf16
                                                      // compute shadow — a third of the all-gather bytes; bias blocks (read in fp32 by the
-                                                     // forward pass) are always pushed; push_master_slices() re-synchronises W on demand
+                                                     // forward pass) are always pushed; push_region_slices() re-synchronises W on demand
+  struct Adam {                                      // fused_allreduce_adam only: the M moment lives in the U region (u_off)
+    long long v_off = -1;                            // second moment region
+    float b1 = 0.9f, b2 = 0.999f, eps = 1e-8f;
+    const unsigned long long* step = nullptr;        // device bias-correction counter: steps taken so far, advanced once per step
+  } adam;
 };
 
 struct ReduceArgs {
@@ -141,11 +146,14 @@ void masked_mean_bwd(const void* dout, const void* mask, void* dh, int Tn, int B
 // ---- comm_kernels.cu
 void sgd_flat(void* W, const void* G, void* U, void* H, const void* block_group, const GroupTable& tab, const void* lr_ptr, float mu,
               int nesterov, float inv_k, long long lo, long long hi, int filter, cudaStream_t st);
+// G: the gradient source (G or R region); filter as sgd_flat; advance = 1: bump the step counter after the update
 void adam_flat(void* W, const void* G, void* M, void* V, void* H, const void* block_group, const GroupTable& tab, const void* lr_ptr, void* step,
-               float b1, float b2, float eps, long long lo, long long hi, cudaStream_t st);
+               float b1, float b2, float eps, long long lo, long long hi, float inv_k, int filter, int advance, cudaStream_t st);
+void adam_advance(void* step, cudaStream_t st);
 void fused_allreduce_sgd(const FusedArgs& a, int algo, int max_blocks, cudaStream_t st);
-// every rank pushes the fp32 master weights of the slice it owns in the two-shot partition of [lo, hi) to all peers
-void push_master_slices(const FusedArgs& a, int max_blocks, cudaStream_t st);
+void fused_allreduce_adam(const FusedArgs& a, int algo, int max_blocks, cudaStream_t st);
+// every rank pushes the slice it owns in the two-shot partition of [lo, hi) of the fp32 region at byte offset `off` to all peers
+void push_region_slices(const FusedArgs& a, long long off, int max_blocks, cudaStream_t st);
 void allreduce_flat(const ReduceArgs& a, int algo, int max_blocks, cudaStream_t st);
 void device_barrier(const CommCtx& c, cudaStream_t st);
 void easgd_elastic(void* w, void* h, void* center, float alpha, long long n, int max_blocks, int lockfree, cudaStream_t st);

@@ -186,8 +186,14 @@ PYBIND11_MODULE(_tmpi_native, m) {
                        ptr_t st) {
     sgd_flat(P(W), P(G), P(U), P(H), P(block_group), make_table(lr_mult, wd, exch), P(lr_ptr), mu, nesterov, inv_k, lo, hi, filter, S(st)); });
   m.def("adam_flat", [](ptr_t W, ptr_t G, ptr_t M, ptr_t V, ptr_t H, ptr_t block_group, std::vector<float> lr_mult, std::vector<float> wd,
-                        std::vector<int> exch, ptr_t lr_ptr, ptr_t step, float b1, float b2, float eps, long long lo, long long hi, ptr_t st) {
-    adam_flat(P(W), P(G), P(M), P(V), P(H), P(block_group), make_table(lr_mult, wd, exch), P(lr_ptr), P(step), b1, b2, eps, lo, hi, S(st)); });
+                        std::vector<int> exch, ptr_t lr_ptr, ptr_t step, float b1, float b2, float eps, long long lo, long long hi, ptr_t st,
+                        float inv_k, int filter, int advance) {
+    adam_flat(P(W), P(G), P(M), P(V), P(H), P(block_group), make_table(lr_mult, wd, exch), P(lr_ptr), P(step), b1, b2, eps, lo, hi, inv_k,
+              filter, advance, S(st)); },
+    py::arg("W"), py::arg("G"), py::arg("M"), py::arg("V"), py::arg("H"), py::arg("block_group"), py::arg("lr_mult"), py::arg("wd"),
+    py::arg("exch"), py::arg("lr_ptr"), py::arg("step"), py::arg("b1"), py::arg("b2"), py::arg("eps"), py::arg("lo"), py::arg("hi"),
+    py::arg("st"), py::arg("inv_k") = 1.f, py::arg("filter") = 0, py::arg("advance") = 1);
+  m.def("adam_advance", [](ptr_t step, ptr_t st) { adam_advance(P(step), S(st)); });
   m.def("easgd_elastic", [](ptr_t w, ptr_t h, ptr_t center, float alpha, long long n, int max_blocks, ptr_t st, int lockfree) {
     easgd_elastic(P(w), P(h), P(center), alpha, n, max_blocks, lockfree, S(st)); },
     py::arg("w"), py::arg("h"), py::arg("center"), py::arg("alpha"), py::arg("n"), py::arg("max_blocks"), py::arg("st"), py::arg("lockfree") = 0);
@@ -248,16 +254,36 @@ PYBIND11_MODULE(_tmpi_native, m) {
            py::arg("lr_mult"), py::arg("wd"), py::arg("exch"), py::arg("lr_ptr"), py::arg("mu"), py::arg("nesterov"), py::arg("inv_k"),
            py::arg("lo"), py::arg("hi"), py::arg("wire16"), py::arg("algo"), py::arg("max_blocks"), py::arg("st"), py::arg("pre_reduced") = 0,
            py::arg("push_master") = 1)
-      .def("push_master_slices",
-           [](PyComm& c, long long w_off, ptr_t block_group, std::vector<float> lr_mult, std::vector<float> wd, std::vector<int> exch,
+      .def("fused_allreduce_adam",
+           [](PyComm& c, long long w_off, long long g_off, long long m_off, long long v_off, long long h_off, long long wire_off,
+              ptr_t block_group, std::vector<float> lr_mult, std::vector<float> wd, std::vector<int> exch, ptr_t lr_ptr, ptr_t step,
+              float b1, float b2, float eps, float inv_k, long long lo, long long hi, int wire16, int algo, int max_blocks, ptr_t st,
+              int push_master) {
+             FusedArgs a;
+             a.pre_reduced = 0;
+             a.push_master = push_master;
+             a.ctx = c.pa->ctx();
+             a.w_off = w_off; a.g_off = g_off; a.u_off = m_off; a.h_off = h_off; a.wire_off = wire_off;
+             a.block_group = (const uint8_t*)P(block_group);
+             a.tab = make_table(lr_mult, wd, exch);
+             a.lr_ptr = (const float*)P(lr_ptr); a.mu = 0.f; a.nesterov = 0; a.inv_k = inv_k; a.lo = lo; a.hi = hi; a.wire16 = wire16;
+             a.adam.v_off = v_off; a.adam.b1 = b1; a.adam.b2 = b2; a.adam.eps = eps;
+             a.adam.step = (const unsigned long long*)P(step);
+             fused_allreduce_adam(a, algo, max_blocks, S(st));
+           }, py::arg("w_off"), py::arg("g_off"), py::arg("m_off"), py::arg("v_off"), py::arg("h_off"), py::arg("wire_off"),
+           py::arg("block_group"), py::arg("lr_mult"), py::arg("wd"), py::arg("exch"), py::arg("lr_ptr"), py::arg("step"), py::arg("b1"),
+           py::arg("b2"), py::arg("eps"), py::arg("inv_k"), py::arg("lo"), py::arg("hi"), py::arg("wire16"), py::arg("algo"),
+           py::arg("max_blocks"), py::arg("st"), py::arg("push_master") = 1)
+      .def("push_region_slices",
+           [](PyComm& c, long long off, ptr_t block_group, std::vector<float> lr_mult, std::vector<float> wd, std::vector<int> exch,
               long long lo, long long hi, int max_blocks, ptr_t st) {
              FusedArgs a;
              a.pre_reduced = 0; a.ctx = c.pa->ctx();
-             a.w_off = w_off; a.g_off = a.u_off = a.wire_off = 0; a.h_off = -1;
+             a.w_off = a.g_off = a.u_off = a.wire_off = 0; a.h_off = -1;
              a.block_group = (const uint8_t*)P(block_group);
              a.tab = make_table(lr_mult, wd, exch);
              a.lr_ptr = nullptr; a.mu = 0.f; a.nesterov = 0; a.inv_k = 1.f; a.lo = lo; a.hi = hi; a.wire16 = 0;
-             push_master_slices(a, max_blocks, S(st));
+             push_region_slices(a, off, max_blocks, S(st));
            })
       .def("configure_gemm_rs", [](PyComm& c, long long g_off) {
              // peer views of the gradient region for the reduce-scatter GEMM epilogue

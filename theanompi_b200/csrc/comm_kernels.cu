@@ -144,31 +144,45 @@ void sgd_flat(void* W, const void* G, void* U, void* H, const void* block_group,
 }
 
 // ============================================================================ flat Adam (Wide-ResNet's optimizer, ref keras_model_zoo/wresnet.py:159)
-// m = b1 m + (1 - b1) g;  v = b2 v + (1 - b2) g^2;  w -= lr * (m / (1 - b1^t)) / (sqrt(v / (1 - b2^t)) + eps), t read from a
-// device counter (the captured CUDA graph keeps counting), lr from device memory, weight decay folded into g, bf16 shadow refreshed.
+// ge = inv_k g + wd w;  m = b1 m + (1 - b1) ge;  v = b2 v + (1 - b2) ge^2;  w -= lr * (m / (1 - b1^t)) / (sqrt(v / (1 - b2^t)) + eps),
+// t read from a device counter (the captured CUDA graph keeps counting), lr from device memory, bf16 shadow refreshed.
+struct AdamHyper { float lr, inv_k, b1, b2, eps, c1, c2; };
+
+__device__ __forceinline__ AdamHyper adam_hyper(const float* lr_ptr, const unsigned long long* step, float inv_k, float b1, float b2,
+                                                float eps) {
+  const float t = (float)(*step + 1ull);
+  return AdamHyper{*lr_ptr, inv_k, b1, b2, eps, 1.f / (1.f - __powf(b1, t)), 1.f / (1.f - __powf(b2, t))};
+}
+
+// __fmul_rn keeps g * inv_k out of FMA contraction: with inv_k = 1 the update rounds exactly as  g + wd * w  does
+__device__ __forceinline__ void adam4(float4& w, float4& m, float4& v, const float4& gsum, const AdamHyper& h, float lrm, float wd) {
+  const float lr = h.lr * lrm;
+#define TMPI_ADAM1(Wc, Mc, Vc, Gc)                                    \
+  {                                                                  \
+    const float ge = __fmul_rn(Gc, h.inv_k) + wd * Wc;               \
+    Mc = h.b1 * Mc + (1.f - h.b1) * ge;                              \
+    Vc = h.b2 * Vc + (1.f - h.b2) * ge * ge;                         \
+    Wc -= lr * (Mc * h.c1) / (sqrtf(Vc * h.c2) + h.eps);             \
+  }
+  TMPI_ADAM1(w.x, m.x, v.x, gsum.x) TMPI_ADAM1(w.y, m.y, v.y, gsum.y) TMPI_ADAM1(w.z, m.z, v.z, gsum.z) TMPI_ADAM1(w.w, m.w, v.w, gsum.w)
+#undef TMPI_ADAM1
+}
+
+// filter: 0 all groups, 1 only non-exchanged (BN) groups, 2 only exchanged groups (as sgd_flat)
 __global__ void __launch_bounds__(kThreads) adam_flat_kernel(float* __restrict__ W, const float* __restrict__ G, float* __restrict__ M,
                                                              float* __restrict__ V, __nv_bfloat16* __restrict__ H,
                                                              const uint8_t* __restrict__ block_group, GroupTable tab,
                                                              const float* __restrict__ lr_ptr, const unsigned long long* __restrict__ step,
-                                                             float b1, float b2, float eps, long long blk_lo, long long blk_hi) {
-  const float t = (float)(*step + 1ull);
-  const float c1 = 1.f / (1.f - __powf(b1, t)), c2 = 1.f / (1.f - __powf(b2, t));
-  const float lr0 = *lr_ptr;
+                                                             float b1, float b2, float eps, float inv_k, long long blk_lo, long long blk_hi,
+                                                             int filter) {
+  const AdamHyper h = adam_hyper(lr_ptr, step, inv_k, b1, b2, eps);
   for (long long b = blk_lo + blockIdx.x; b < blk_hi; b += gridDim.x) {
     const int g = block_group[b];
-    const float lr = lr0 * tab.lr_mult[g], wd = tab.wd[g];
+    if ((filter == 1 && tab.exch[g]) || (filter == 2 && !tab.exch[g])) continue;
     const long long i = b * kArenaBlock + threadIdx.x * 4;
     float4 w = *reinterpret_cast<const float4*>(W + i), m = *reinterpret_cast<const float4*>(M + i), v = *reinterpret_cast<const float4*>(V + i);
     const float4 gg = *reinterpret_cast<const float4*>(G + i);
-#define TMPI_ADAM1(Wc, Mc, Vc, Gc)                                    \
-  {                                                                  \
-    const float ge = Gc + wd * Wc;                                   \
-    Mc = b1 * Mc + (1.f - b1) * ge;                                  \
-    Vc = b2 * Vc + (1.f - b2) * ge * ge;                             \
-    Wc -= lr * (Mc * c1) / (sqrtf(Vc * c2) + eps);                   \
-  }
-    TMPI_ADAM1(w.x, m.x, v.x, gg.x) TMPI_ADAM1(w.y, m.y, v.y, gg.y) TMPI_ADAM1(w.z, m.z, v.z, gg.z) TMPI_ADAM1(w.w, m.w, v.w, gg.w)
-#undef TMPI_ADAM1
+    adam4(w, m, v, gg, h, tab.lr_mult[g], tab.wd[g]);
     *reinterpret_cast<float4*>(W + i) = w;
     *reinterpret_cast<float4*>(M + i) = m;
     *reinterpret_cast<float4*>(V + i) = v;
@@ -177,30 +191,65 @@ __global__ void __launch_bounds__(kThreads) adam_flat_kernel(float* __restrict__
 }
 __global__ void adam_advance_kernel(unsigned long long* step) { if (threadIdx.x == 0 && blockIdx.x == 0) *step += 1ull; }
 
+void adam_advance(void* step, cudaStream_t st) {
+  adam_advance_kernel<<<1, 32, 0, st>>>((unsigned long long*)step);
+  count_launch(); TMPI_CHECK_LAUNCH("adam_advance"); ::tmpi::check_capture(st, "adam_advance");
+}
+
 void adam_flat(void* W, const void* G, void* M, void* V, void* H, const void* block_group, const GroupTable& tab, const void* lr_ptr, void* step,
-               float b1, float b2, float eps, long long lo, long long hi, cudaStream_t st) {
+               float b1, float b2, float eps, long long lo, long long hi, float inv_k, int filter, int advance, cudaStream_t st) {
   if (lo % kArenaBlock || hi % kArenaBlock) throw std::runtime_error("adam_flat: range must be block aligned");
   const long long nb = (hi - lo) / kArenaBlock;
-  if (nb <= 0) return;
-  int grid = (int)std::min<long long>(nb, (long long)sm_count() * 8);
-  adam_flat_kernel<<<grid, kThreads, 0, st>>>((float*)W, (const float*)G, (float*)M, (float*)V, (__nv_bfloat16*)H, (const uint8_t*)block_group, tab,
-                                              (const float*)lr_ptr, (const unsigned long long*)step, b1, b2, eps, lo / kArenaBlock, hi / kArenaBlock);
-  adam_advance_kernel<<<1, 32, 0, st>>>((unsigned long long*)step);
-  count_launch(2); TMPI_CHECK_LAUNCH("adam_flat"); ::tmpi::check_capture(st, "adam_flat");
+  if (nb > 0) {
+    int grid = (int)std::min<long long>(nb, (long long)sm_count() * 8);
+    adam_flat_kernel<<<grid, kThreads, 0, st>>>((float*)W, (const float*)G, (float*)M, (float*)V, (__nv_bfloat16*)H, (const uint8_t*)block_group,
+                                                tab, (const float*)lr_ptr, (const unsigned long long*)step, b1, b2, eps, inv_k, lo / kArenaBlock,
+                                                hi / kArenaBlock, filter);
+    count_launch(); TMPI_CHECK_LAUNCH("adam_flat"); ::tmpi::check_capture(st, "adam_flat");
+  }
+  if (advance) adam_advance(step, st);
 }
 
 // ============================================================================ fused collectives
-__device__ __forceinline__ void local_block_update(const FusedArgs& a, const Hyper& h, long long b, int g) {
+// The per-element update is a compile-time policy of the fused kernels: Rule::hyper() reads the step's hyper-parameters once per
+// CTA, Rule::update() applies the rule to one float4 of W given the gradient sum, reading and writing the rule's own state (U for
+// momentum SGD; M = U region and V for Adam) at element i of the calling rank's arena.
+struct SgdRule {
+  typedef Hyper Hp;
+  static __device__ __forceinline__ Hyper hyper(const FusedArgs& a) { return Hyper{*a.lr_ptr, a.mu, a.inv_k, a.nesterov}; }
+  static __device__ __forceinline__ void update(const FusedArgs& a, const Hyper& h, long long i, float4& w, const float4& gsum, int g) {
+    float* U = region<float>(a.ctx, a.ctx.rank, a.u_off) + i;
+    float4 u = *reinterpret_cast<const float4*>(U);
+    sgd4(w, u, gsum, h, a.tab.lr_mult[g], a.tab.wd[g]);
+    *reinterpret_cast<float4*>(U) = u;
+  }
+};
+struct AdamRule {
+  typedef AdamHyper Hp;
+  static __device__ __forceinline__ AdamHyper hyper(const FusedArgs& a) {
+    return adam_hyper(a.lr_ptr, a.adam.step, a.inv_k, a.adam.b1, a.adam.b2, a.adam.eps);
+  }
+  static __device__ __forceinline__ void update(const FusedArgs& a, const AdamHyper& h, long long i, float4& w, const float4& gsum, int g) {
+    float* M = region<float>(a.ctx, a.ctx.rank, a.u_off) + i;
+    float* V = region<float>(a.ctx, a.ctx.rank, a.adam.v_off) + i;
+    float4 m = *reinterpret_cast<const float4*>(M), v = *reinterpret_cast<const float4*>(V);
+    adam4(w, m, v, gsum, h, a.tab.lr_mult[g], a.tab.wd[g]);
+    *reinterpret_cast<float4*>(M) = m;
+    *reinterpret_cast<float4*>(V) = v;
+  }
+};
+
+// non-exchanged (BN) block: the rank's own gradient, no averaging
+template <class Rule>
+__device__ __forceinline__ void local_block_update(const FusedArgs& a, const typename Rule::Hp& h, long long b, int g) {
   const long long i = b * kArenaBlock + threadIdx.x * 4;
   float* W = region<float>(a.ctx, a.ctx.rank, a.w_off);
-  float* U = region<float>(a.ctx, a.ctx.rank, a.u_off);
   const float* G = region<float>(a.ctx, a.ctx.rank, a.g_off);
-  float4 w = *reinterpret_cast<const float4*>(W + i), u = *reinterpret_cast<const float4*>(U + i);
+  float4 w = *reinterpret_cast<const float4*>(W + i);
   const float4 gg = *reinterpret_cast<const float4*>(G + i);
-  Hyper hl = h; hl.inv_k = 1.f;
-  sgd4(w, u, gg, hl, a.tab.lr_mult[g], a.tab.wd[g]);
+  typename Rule::Hp hl = h; hl.inv_k = 1.f;
+  Rule::update(a, hl, i, w, gg, g);
   *reinterpret_cast<float4*>(W + i) = w;
-  *reinterpret_cast<float4*>(U + i) = u;
   if (a.h_off >= 0) *reinterpret_cast<uint2*>(region<__nv_bfloat16>(a.ctx, a.ctx.rank, a.h_off) + i) = pack_bf16x4(w);
 }
 
@@ -232,9 +281,9 @@ __device__ __forceinline__ float4 gather_grad(const FusedArgs& a, long long i) {
 // ---- one-shot: every rank reduces every block itself
 // U arena blocks are in flight per CTA iteration (U x world independent 16 B peer loads per thread) — a single
 // load per thread cannot cover the ~2 us NVLink round trip.
-template <int U>
-__global__ void __launch_bounds__(kThreads) fused_oneshot_sgd_kernel(const FusedArgs a) {
-  const Hyper h{*a.lr_ptr, a.mu, a.inv_k, a.nesterov};
+template <class Rule, int U>
+__global__ void __launch_bounds__(kThreads) fused_oneshot_kernel(const FusedArgs a) {
+  const typename Rule::Hp h = Rule::hyper(a);
   const long long blo = a.lo / kArenaBlock, bhi = a.hi / kArenaBlock;
   if (a.wire16) {
     for (long long b = blo + blockIdx.x; b < bhi; b += gridDim.x)
@@ -242,7 +291,6 @@ __global__ void __launch_bounds__(kThreads) fused_oneshot_sgd_kernel(const Fused
   }
   block_barrier(a.ctx);                                  // peers' gradients (or wire copies) are complete
   float* W = region<float>(a.ctx, a.ctx.rank, a.w_off);
-  float* U_ = region<float>(a.ctx, a.ctx.rank, a.u_off);
   for (long long b0 = blo + blockIdx.x; b0 < bhi; b0 += (long long)gridDim.x * U) {
     float4 gs[U]; int grp[U]; bool ex[U];
 #pragma unroll
@@ -256,12 +304,11 @@ __global__ void __launch_bounds__(kThreads) fused_oneshot_sgd_kernel(const Fused
     for (int u = 0; u < U; ++u) {
       const long long b = b0 + (long long)u * gridDim.x;
       if (grp[u] < 0) continue;
-      if (!ex[u]) { local_block_update(a, h, b, grp[u]); continue; }
+      if (!ex[u]) { local_block_update<Rule>(a, h, b, grp[u]); continue; }
       const long long i = b * kArenaBlock + threadIdx.x * 4;
-      float4 w = *reinterpret_cast<const float4*>(W + i), uu = *reinterpret_cast<const float4*>(U_ + i);
-      sgd4(w, uu, gs[u], h, a.tab.lr_mult[grp[u]], a.tab.wd[grp[u]]);
+      float4 w = *reinterpret_cast<const float4*>(W + i);
+      Rule::update(a, h, i, w, gs[u], grp[u]);
       *reinterpret_cast<float4*>(W + i) = w;
-      *reinterpret_cast<float4*>(U_ + i) = uu;
       if (a.h_off >= 0) *reinterpret_cast<uint2*>(region<__nv_bfloat16>(a.ctx, a.ctx.rank, a.h_off) + i) = pack_bf16x4(w);
     }
   }
@@ -269,9 +316,9 @@ __global__ void __launch_bounds__(kThreads) fused_oneshot_sgd_kernel(const Fused
 }
 
 // ---- two-shot: rank r owns a contiguous slice of the range; reduce → update → push W (+H) to every peer
-template <int U>
-__global__ void __launch_bounds__(kThreads) fused_twoshot_sgd_kernel(const FusedArgs a, int use_nvls) {
-  const Hyper h{*a.lr_ptr, a.mu, a.inv_k, a.nesterov};
+template <class Rule, int U>
+__global__ void __launch_bounds__(kThreads) fused_twoshot_kernel(const FusedArgs a, int use_nvls) {
+  const typename Rule::Hp h = Rule::hyper(a);
   const long long blo = a.lo / kArenaBlock, bhi = a.hi / kArenaBlock;
   const long long nb = bhi - blo;
   const long long per = (nb + a.ctx.world - 1) / a.ctx.world;
@@ -287,7 +334,6 @@ __global__ void __launch_bounds__(kThreads) fused_twoshot_sgd_kernel(const Fused
   block_barrier(a.ctx);
   const long long s0 = blo + R * per, s1 = min(bhi, s0 + per);
   float* W = region<float>(a.ctx, R, a.w_off);
-  float* U_ = region<float>(a.ctx, R, a.u_off);
   for (long long b0 = s0 + blockIdx.x; b0 < s1; b0 += (long long)gridDim.x * U) {
     float4 gs[U]; int grp[U];
 #pragma unroll
@@ -317,9 +363,8 @@ __global__ void __launch_bounds__(kThreads) fused_twoshot_sgd_kernel(const Fused
       if (grp[u] < 0) continue;
       const long long b = b0 + (long long)u * gridDim.x;
       const long long i = b * kArenaBlock + threadIdx.x * 4;
-      float4 w = *reinterpret_cast<const float4*>(W + i), uu = *reinterpret_cast<const float4*>(U_ + i);
-      sgd4(w, uu, gs[u], h, a.tab.lr_mult[grp[u]], a.tab.wd[grp[u]]);
-      *reinterpret_cast<float4*>(U_ + i) = uu;
+      float4 w = *reinterpret_cast<const float4*>(W + i);
+      Rule::update(a, h, i, w, gs[u], grp[u]);
       const uint2 wh = pack_bf16x4(w);
       // owner-keeps-master ships only the bf16 shadow — of plain WEIGHT blocks (group 0).  Biases (and anything else the
       // forward pass reads in fp32 straight from W) always travel as fp32 masters: they are a few KB.
@@ -342,7 +387,7 @@ __global__ void __launch_bounds__(kThreads) fused_twoshot_sgd_kernel(const Fused
   // non-exchanged (BN) blocks: every rank updates all of them locally
   for (long long b = blo + blockIdx.x; b < bhi; b += gridDim.x) {
     const int g = a.block_group[b];
-    if (!a.tab.exch[g]) local_block_update(a, h, b, g);
+    if (!a.tab.exch[g]) local_block_update<Rule>(a, h, b, g);
   }
   block_barrier(a.ctx);                                  // pushed weights are visible everywhere
 }
@@ -355,16 +400,17 @@ static int pick_grid(long long nblocks, int max_blocks) {
 }
 
 // algo: 0 one-shot, 1 two-shot (P2P), 2 two-shot NVLS
-void fused_allreduce_sgd(const FusedArgs& a, int algo, int max_blocks, cudaStream_t st) {
-  if (a.lo % kArenaBlock || a.hi % kArenaBlock) throw std::runtime_error("fused_allreduce_sgd: range must be block aligned");
+template <class Rule>
+static void fused_allreduce(const FusedArgs& a, int algo, int max_blocks, cudaStream_t st, const char* name) {
+  if (a.lo % kArenaBlock || a.hi % kArenaBlock) throw std::runtime_error(std::string(name) + ": range must be block aligned");
   const long long nb = (a.hi - a.lo) / kArenaBlock;
   if (nb <= 0) return;
-  if (algo == 2 && a.ctx.mc_arena == nullptr) throw std::runtime_error("fused_allreduce_sgd: NVLS requested without a multicast mapping");
+  if (algo == 2 && a.ctx.mc_arena == nullptr) throw std::runtime_error(std::string(name) + ": NVLS requested without a multicast mapping");
   const bool wide = a.ctx.world > 4;                     // keep (U x world) peer loads per thread around 8..16
   if (a.pre_reduced && algo == 0) algo = a.ctx.mc_arena ? 2 : 1;     // ownership is the two-shot partition
   if (algo == 0) {
-    if (wide) fused_oneshot_sgd_kernel<2><<<pick_grid(nb, max_blocks), kThreads, 0, st>>>(a);
-    else fused_oneshot_sgd_kernel<4><<<pick_grid(nb, max_blocks), kThreads, 0, st>>>(a);
+    if (wide) fused_oneshot_kernel<Rule, 2><<<pick_grid(nb, max_blocks), kThreads, 0, st>>>(a);
+    else fused_oneshot_kernel<Rule, 4><<<pick_grid(nb, max_blocks), kThreads, 0, st>>>(a);
   } else {
     const long long per = (nb + a.ctx.world - 1) / a.ctx.world;
     const int nv = algo == 2 ? 1 : 0;
@@ -374,39 +420,50 @@ void fused_allreduce_sgd(const FusedArgs& a, int algo, int max_blocks, cudaStrea
     static const int u_env = [] { const char* e = getenv("TMPI_FUSED_U"); return e ? atoi(e) : 0; }();
     int U = nv ? 8 : (a.ctx.world <= 2 ? 8 : (wide ? 2 : 4));
     if (u_env == 2 || u_env == 4 || u_env == 8) U = u_env;
-    if (U == 8) fused_twoshot_sgd_kernel<8><<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, nv);
-    else if (U == 4) fused_twoshot_sgd_kernel<4><<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, nv);
-    else fused_twoshot_sgd_kernel<2><<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, nv);
+    if (U == 8) fused_twoshot_kernel<Rule, 8><<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, nv);
+    else if (U == 4) fused_twoshot_kernel<Rule, 4><<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, nv);
+    else fused_twoshot_kernel<Rule, 2><<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, nv);
   }
-  count_launch(); TMPI_CHECK_LAUNCH("fused_allreduce_sgd"); ::tmpi::check_capture(st, "fused_allreduce_sgd");
+  count_launch(); TMPI_CHECK_LAUNCH(name); ::tmpi::check_capture(st, name);
 }
 
-// every rank pushes the fp32 master of the slice it owns (two-shot partition of [lo, hi)) to all peers: re-synchronises W after
-// steps that ran with push_master = 0 (before a checkpoint / weight averaging / anything that reads W on a non-owner)
-__global__ void __launch_bounds__(kThreads) push_master_kernel(const FusedArgs a) {
+void fused_allreduce_sgd(const FusedArgs& a, int algo, int max_blocks, cudaStream_t st) {
+  fused_allreduce<SgdRule>(a, algo, max_blocks, st, "fused_allreduce_sgd");
+}
+
+void fused_allreduce_adam(const FusedArgs& a, int algo, int max_blocks, cudaStream_t st) {
+  if (a.pre_reduced) throw std::runtime_error("fused_allreduce_adam: gradients reduce-scattered by the GEMM epilogue are not supported");
+  if (a.adam.step == nullptr) throw std::runtime_error("fused_allreduce_adam: no step counter");
+  fused_allreduce<AdamRule>(a, algo, max_blocks, st, "fused_allreduce_adam");
+}
+
+// every rank pushes the slice it owns (two-shot partition of [lo, hi)) of the fp32 region at byte offset `off` to all peers:
+// re-synchronises W after steps that ran with push_master = 0, and the optimizer state (momentum / Adam moments) that two-shot
+// steps update on the owner only (before a checkpoint / weight averaging / anything that reads them on a non-owner)
+__global__ void __launch_bounds__(kThreads) push_region_kernel(const FusedArgs a, long long off) {
   const long long blo = a.lo / kArenaBlock, bhi = a.hi / kArenaBlock;
   const long long per = (bhi - blo + a.ctx.world - 1) / a.ctx.world;
   const int R = a.ctx.rank;
   const long long s0 = blo + R * per, s1 = min(bhi, s0 + per);
   block_barrier(a.ctx);
-  const float* W = region<float>(a.ctx, R, a.w_off);
+  const float* X = region<float>(a.ctx, R, off);
   for (long long b = s0 + blockIdx.x; b < s1; b += gridDim.x) {
     if (!a.tab.exch[a.block_group[b]]) continue;
     const long long i = b * kArenaBlock + threadIdx.x * 4;
-    const float4 w = *reinterpret_cast<const float4*>(W + i);
+    const float4 x = *reinterpret_cast<const float4*>(X + i);
 #pragma unroll
     for (int p = 0; p < kMaxRanks; ++p)
-      if (p < a.ctx.world && p != R) st_f4(region<float>(a.ctx, p, a.w_off) + i, w);
+      if (p < a.ctx.world && p != R) st_f4(region<float>(a.ctx, p, off) + i, x);
   }
   block_barrier(a.ctx);
 }
-void push_master_slices(const FusedArgs& a, int max_blocks, cudaStream_t st) {
-  if (a.lo % kArenaBlock || a.hi % kArenaBlock) throw std::runtime_error("push_master_slices: range must be block aligned");
+void push_region_slices(const FusedArgs& a, long long off, int max_blocks, cudaStream_t st) {
+  if (a.lo % kArenaBlock || a.hi % kArenaBlock) throw std::runtime_error("push_region_slices: range must be block aligned");
   const long long nb = (a.hi - a.lo) / kArenaBlock;
   if (nb <= 0) return;
   const long long per = (nb + a.ctx.world - 1) / a.ctx.world;
-  push_master_kernel<<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a);
-  count_launch(); TMPI_CHECK_LAUNCH("push_master_slices"); ::tmpi::check_capture(st, "push_master_slices");
+  push_region_kernel<<<pick_grid(per, max_blocks), kThreads, 0, st>>>(a, off);
+  count_launch(); TMPI_CHECK_LAUNCH("push_region_slices"); ::tmpi::check_capture(st, "push_region_slices");
 }
 
 // ============================================================================ plain flat allreduce (sum * scale) src region → dst region

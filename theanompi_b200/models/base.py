@@ -29,7 +29,7 @@ import torch
 from .. import ops
 from ..parallel.arena import FlatArena
 from ..utils import nvtx
-from ..utils.opt import FlatSGD, SharedScalar, pre_model_iter_fn
+from ..utils.opt import FlatAdam, FlatSGD, SharedScalar, pre_model_iter_fn
 from .layers2 import BatchNormal, Crop, Dropout, count_params
 
 
@@ -61,12 +61,18 @@ class ModelBase(object):
     rand_crop = True
     monitor_grad = False
     bias_lr_mult = 2.0             # biases train with 2x lr in the reference's optimizer (lib/opt.py:181-268)
+    optimizer = "msgd"             # update rule of the arena: 'msgd' (momentum SGD, lib/opt.py) or 'adam'; config['optimizer'] overrides
     graph_safe = True              # False: the step draws host-side randomness / has host control flow → never auto-capture
     name = "Model"
 
     def __init__(self, config):
         self.config = config
         self.verbose = config.get("verbose", False)
+        opt = config.get("optimizer", self.optimizer)
+        opt = "msgd" if opt == "sgd" else opt
+        if opt not in ("msgd", "adam"):
+            raise ValueError("optimizer must be 'msgd' or 'adam', got %r" % (opt,))
+        self.optimizer = opt
         self.rank = config.get("rank", 0)
         self.size = config.get("size", 1)
         self.no_paraload = config.get("no_paraload", False)
@@ -125,9 +131,10 @@ class ModelBase(object):
         allocator = self.config.get("arena_allocator")
         self.arena = FlatArena(self.params, self.weight_types, self.device, weight_decay=self.eta, bias_lr_mult=self.bias_lr_mult,
                                with_recv=allocator is not None, allocator=allocator,
-                               shadow=False if self.precision == "tf32" else self.config.get("_arena_shadow"))
+                               shadow=False if self.precision == "tf32" else self.config.get("_arena_shadow"), optimizer=self.optimizer)
         self.shared_lr = SharedScalar(self.arena.hyper, 0, self.base_lr)
         self.sgd = FlatSGD(self.arena, self.mu, self.use_nesterov_momentum, self.use_momentum)
+        self.adam = FlatAdam(self.arena) if self.optimizer == "adam" else None
         B = self.batch_size
         fb = self.file_batch_size
         self.input_shape = tuple(input_shape)           # (B, H, W, C)

@@ -1,7 +1,9 @@
 """Wide-ResNet WRN-28-4 on CIFAR-10 with Adam (ref ``keras_model_zoo/wresnet.py:37-82,159``):
-pre-activation blocks, widths (16, 64, 128, 256), 4 blocks per group.  Self-contained
-optimizer ⇒ only ``sync_type='avg'`` (``:152-153``); params = all trainable weights
-(``:257-263``).  The model of the GOSGD benchmark config (BASELINE.json).
+pre-activation blocks, widths (16, 64, 128, 256), 4 blocks per group; params = all trainable
+weights (``:257-263``).  The model of the GOSGD benchmark config (BASELINE.json).  The reference
+only averages weights (``sync_type='avg'``, ``:152-153``); here ``'cdd'`` also works: gradients are
+averaged across ranks, then one Adam step (inside the fused exchange kernels, or after a classic
+strategy's all-reduce).
 
 ``Wide_ResNet`` runs on the hand-written sm_100a kernels (tcgen05 implicit-GEMM convolutions, fused BatchNormal+ReLU, native
 residual add, one flat Adam kernel; CUDA-graph captured step).  ``Wide_ResNetTorch`` is the same network on torch modules
@@ -59,6 +61,7 @@ class WRN(nn.Module):
 class Wide_ResNet(ModelBase):
     n_epochs, batch_size, file_batch_size, learning_rate = n_epochs, batch_size, file_batch_size, learning_rate
     weight_decay, momentum = 0.0, 0.9
+    optimizer = "adam"             # config['optimizer'] = 'sgd' / 'msgd' trains with momentum SGD instead
     bias_lr_mult = 1.0             # Adam: one learning rate for every parameter
     lr_policy = "step"
     lr_step = [60, 120, 160]
@@ -148,32 +151,9 @@ class Wide_ResNet(ModelBase):
         bn, gap, flat, sm = self.head
         return sm.forward(flat.forward(gap.forward(bn.forward(x))))
 
-    def compile_iter_fns(self, sync_type="avg", aggregate="momentum", fused_tail=None):
-        """Adam is self-contained (ref ``wresnet.py:152-159``): weights are averaged across workers (``sync_type='avg'``)."""
-        if self.config.get("optimizer", "adam") == "sgd":
-            return super().compile_iter_fns(sync_type, aggregate, fused_tail)
-        if sync_type != "avg" and self.size > 1:
-            raise ValueError("Wide_ResNet trains with Adam: only sync_type='avg' is supported (as in the reference, wresnet.py:152-153)")
-        from ...utils.opt import FlatAdam
-        self.sync_type = "avg"
-        self.adam = FlatAdam(self.arena)
-        self.set_step_tail(lambda: self.adam.step())
-        self.get_vel = lambda subb=0: self.forward_backward(subb)
-        self.descent_vel = lambda: None
-        self.train_iter_fn = self.get_vel
-        self.vels, self.vels2 = [], []
-        self.compile_val()
-        self.val_iter_fn = self.val_fn
-
-    def extra_state(self):
-        sd = super().extra_state()
-        if getattr(self, "adam", None) is not None:
-            sd["adam"] = self.adam.state_dict()
-        return sd
-
     def load_extra_state(self, sd):
         super().load_extra_state(sd)
-        if "adam" in sd and getattr(self, "adam", None) is not None:
+        if "adam" in sd and self.adam is not None:      # checkpoints written before the moments moved into the arena
             self.adam.load_state_dict(sd["adam"])
 
 

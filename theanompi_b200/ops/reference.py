@@ -161,6 +161,25 @@ def sgd_flat(w, g, u, lr_mult, wd, lr, mu, nesterov, inv_k, w_half=None):
     return w, u
 
 
+def adam_flat(w, g, m, v, lr_mult, wd, lr, b1, b2, eps, t, inv_k=1.0, w_half=None):
+    """One Adam step (step number ``t`` >= 1) over flat fp32 buffers with per-element ``lr_mult`` / ``wd`` vectors, as the
+    native ``adam_flat`` / fused Adam kernels compute it:
+
+        ge = g * inv_k + wd * w
+        m  = b1 * m + (1 - b1) * ge
+        v  = b2 * v + (1 - b2) * ge^2
+        w -= lr * lr_mult * (m / (1 - b1^t)) / (sqrt(v / (1 - b2^t)) + eps)
+    """
+    ge = g * inv_k + wd * w
+    m.mul_(b1).add_(ge, alpha=1 - b1)
+    v.mul_(b2).addcmul_(ge, ge, value=1 - b2)
+    mh, vh = m / (1 - b1 ** t), v / (1 - b2 ** t)
+    w.sub_(lr * lr_mult * mh / (vh.sqrt() + eps))
+    if w_half is not None:
+        w_half.copy_(w)
+    return w, m, v
+
+
 def easgd_elastic(w, c, alpha):
     """EASGD elastic move (ref ``exchanger.py:188-211``) with both sides updated
     from the SAME difference: ``d = alpha (w - c); w -= d; c += d``."""

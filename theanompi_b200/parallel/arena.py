@@ -12,6 +12,7 @@ contiguous fp32 regions of ONE allocation:
     U  momentum
     R  receive buffer        (``model.vels2`` views; only classic strategies use it)
     H  bf16 compute shadow of W (GPU only; written by the fused update kernel)
+    V  Adam second moment    (``optimizer='adam'`` only; U then holds the first moment)
 
 so that optimizer + collective become one or a few launches over a flat range,
 and — when the allocation comes from the peer-mapped symmetric allocator
@@ -51,7 +52,7 @@ def default_group(name, weight_type):
 class FlatArena(object):
     def __init__(self, params, weight_types=None, device=None, weight_decay=0.0,
                  shadow=None, with_recv=False, allocator=None, bias_lr_mult=2.0,
-                 exchange_bn=False):
+                 exchange_bn=False, optimizer="msgd"):
         self.params = list(params)
         n = len(self.params)
         if weight_types is None:
@@ -69,6 +70,7 @@ class FlatArena(object):
         self.n_real = sum(self.sizes)
         self.use_shadow = (self.device.type == "cuda") if shadow is None else bool(shadow)
         self.allocator = allocator
+        self.optimizer = optimizer
 
         # ---- group table
         self.group_of = [default_group(getattr(p, "pname", None), wt)
@@ -99,6 +101,9 @@ class FlatArena(object):
         if self.use_shadow:
             layout["H"] = nbytes
             nbytes += self.numel * 2
+        if optimizer == "adam":                 # after H: SGD arenas keep their layout
+            layout["V"] = nbytes
+            nbytes += self.numel * 4
         self.nbytes = nbytes
         self.layout = layout
         if allocator is not None:
@@ -112,6 +117,9 @@ class FlatArena(object):
         if self.use_shadow:
             self._regions["H"] = self.raw[layout["H"]:layout["H"] + self.numel * 2].view(torch.bfloat16)
             self._regions["H"].zero_()
+        if "V" in layout:
+            self._regions["V"] = self.raw[layout["V"]:layout["V"] + self.numel * 4].view(torch.float32)
+            self._regions["V"].zero_()
 
         dev = self.device
         self.block_group = torch.from_numpy(bg).to(dev)
@@ -121,6 +129,8 @@ class FlatArena(object):
         # hyper-parameters live on the device so CUDA graphs never need re-capture:
         # [lr, mu, inv_k, nesterov_flag]
         self.hyper = torch.zeros(8, dtype=torch.float32, device=dev)
+        # Adam bias-correction counter: optimizer steps taken so far (device memory, advanced once per step inside the graph)
+        self.adam_t = torch.zeros(1, dtype=torch.int64, device=dev) if optimizer == "adam" else None
         self._bind()
 
     # ------------------------------------------------------------------ regions
@@ -139,6 +149,18 @@ class FlatArena(object):
     @property
     def H(self):
         return self._regions.get("H")
+
+    @property
+    def V(self):
+        return self._regions.get("V")
+
+    def ensure_adam_state(self):
+        """V region + step counter of an arena built for another optimizer (a plain local buffer outside the allocation, like
+        a late ``R``): enough for the local :class:`FlatAdam` step, not for the fused exchange."""
+        if "V" not in self._regions:
+            self._regions["V"] = torch.zeros(self.numel, dtype=torch.float32, device=self.device)
+        if self.adam_t is None:
+            self.adam_t = torch.zeros(1, dtype=torch.int64, device=self.device)
 
     @property
     def R(self):
@@ -237,12 +259,19 @@ class FlatArena(object):
 
     # ------------------------------------------------------------------ checkpoint
     def state_dict(self):
-        return {"W": self.W.detach().cpu().clone(), "U": self.U.detach().cpu().clone(),
-                "offsets": list(self.offsets), "sizes": list(self.sizes)}
+        sd = {"W": self.W.detach().cpu().clone(), "U": self.U.detach().cpu().clone(),
+              "offsets": list(self.offsets), "sizes": list(self.sizes)}
+        if self.V is not None:
+            sd["V"] = self.V.detach().cpu().clone()
+            sd["t"] = int(self.adam_t)
+        return sd
 
     def load_state_dict(self, sd):
         assert list(sd["sizes"]) == list(self.sizes), "arena layout mismatch"
         with torch.no_grad():
             self.W.copy_(sd["W"].to(self.device))
             self.U.copy_(sd["U"].to(self.device))
+            if self.V is not None and "V" in sd:
+                self.V.copy_(sd["V"].to(self.device))
+                self.adam_t.fill_(int(sd["t"]))
         self.refresh_shadow()

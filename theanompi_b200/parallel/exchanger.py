@@ -9,7 +9,8 @@
 B200-native hot paths (no NCCL / MPI call on them):
 
 * BSP ``fused*`` strategies: ONE kernel family reads all peers' gradients over NVLink,
-  averages, applies weight-decay + momentum + lr, refreshes the bf16 compute shadow and
+  averages, applies the model's update rule (weight-decay + momentum + lr, or Adam),
+  refreshes the bf16 compute shadow and
   (two-shot / NVLS) pushes the updated slice to the peers; launched per bucket on a side
   stream from the backward's grad-ready callbacks so it overlaps backward; part of the
   captured CUDA graph.
@@ -82,6 +83,10 @@ class BSP_Exchanger(object):
         if self.fused:
             if sync_type != "cdd":
                 raise ValueError("fused strategies implement the cdd (gradient) exchange")
+            self.adam = getattr(model, "optimizer", "msgd") == "adam"
+            if self.adam and exch_strategy == "fused_rs":
+                raise ValueError("fused_rs (gradients reduce-scattered by the GEMM epilogue) supports momentum SGD only, not Adam; "
+                                 "use fused or fused16")
             if gpucomm is None:
                 raise RuntimeError("strategy %s needs the symmetric peer arena (GPUs of one node)" % exch_strategy)
             self.algo, self.wire16 = FUSED[exch_strategy]
@@ -187,6 +192,13 @@ class BSP_Exchanger(object):
         if blocks is None and self.overlap:
             big = int(os.environ.get("TMPI_OVERLAP_BLOCKS", "64"))     # measured at 2 ranks: 16 → 4.5 ms, 32 → 3.1, 64 → 2.17, 148 → 2.28
             blocks = big if (b["hi"] - b["lo"]) * 4 > (8 << 20) else min(8, big)
+        if self.adam:
+            # Adam: two-shot buckets update the moments on the owner of a slice only → sync_master() pushes them too
+            ad = m.adam
+            self.gpucomm.fused_allreduce_adam(self.arena, b["lo"], b["hi"], ad.b1, ad.b2, ad.eps, algo=self.algo, wire16=self.wire16,
+                                              max_blocks=blocks, push_master=self.push_master)
+            self._master_stale = True
+            return
         self.gpucomm.fused_allreduce_sgd(self.arena, b["lo"], b["hi"], mu, m.use_nesterov_momentum,
                                          algo=self.algo, wire16=self.wire16, max_blocks=blocks, pre_reduced=b.get("rs", False),
                                          push_master=self.push_master)
@@ -194,14 +206,19 @@ class BSP_Exchanger(object):
             self._master_stale = True
 
     def sync_master(self):
-        """Collective: make every rank's fp32 master weights current again (owner-keeps-master mode).  Buckets that ran the
-        one-shot algorithm are already identical everywhere; the two-shot ones push their owner slices."""
-        if not getattr(self, "fused", False) or self.push_master or not self._master_stale:
+        """Collective: make every rank's fp32 master weights (owner-keeps-master mode) and, for Adam, both moments current
+        again.  Buckets that ran the one-shot algorithm are already identical everywhere; the two-shot ones push their owner
+        slices."""
+        if not getattr(self, "fused", False) or not self._master_stale:
+            return
+        regions = ([] if self.push_master else ["W"]) + (["U", "V"] if self.adam else [])
+        if not regions:
             return
         for b in self.buckets:
             nbytes = (b["hi"] - b["lo"]) * (2 if self.wire16 else 4)
             if self.gpucomm.pick_algo(nbytes, self.algo) != 0 or b.get("rs", False):
-                self.gpucomm.push_master_slices(self.arena, b["lo"], b["hi"])
+                for r in regions:
+                    self.gpucomm.push_region_slices(self.arena, r, b["lo"], b["hi"])
         torch.cuda.synchronize(self.arena.device)
         self.comm.Barrier()
         self._master_stale = False
@@ -233,6 +250,9 @@ class BSP_Exchanger(object):
         else:
             for bi in range(len(self.buckets)):                   # one bucket, or solo reduce-scatter buckets + the rest
                 self._launch_bucket(bi)
+        if self.adam:
+            # every bucket of this step read the same t; the next step's first bucket waits on this stream
+            self.gpucomm.adam_advance(self.arena)
 
     # ------------------------------------------------------------------ the per-iteration call
     def exchange(self, recorder):

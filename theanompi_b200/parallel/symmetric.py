@@ -207,13 +207,41 @@ class SymmetricComm(object):
                                     int(bool(pre_reduced)), int(bool(push_master)))
         return a
 
+    def fused_allreduce_adam(self, arena, lo, hi, b1, b2, eps, inv_k=None, algo="auto", wire16=False, max_blocks=None,
+                             push_master=True):
+        """Average the ranks' gradients of ``[lo, hi)`` and take one Adam step (moments in the arena's U and V regions, step
+        counter ``arena.adam_t``, which this call reads but does not advance: the caller advances it once per optimizer step
+        with :meth:`adam_advance`).  Same algorithms, wire formats and owner-keeps-master mode as :meth:`fused_allreduce_sgd`;
+        two-shot updates the moments on the owner of a slice only (:meth:`push_region_slices` re-synchronises them)."""
+        from ..ops.cuda_impl import _table
+        if "V" not in arena.layout:
+            raise ValueError("fused Adam needs an arena built with optimizer='adam' (V region in the symmetric allocation)")
+        lrm, wd, ex = _table(arena)
+        h_off = arena.layout["H"] if arena.H is not None else -1
+        a = self.pick_algo((hi - lo) * (2 if wire16 else 4), algo)
+        self.pa.fused_allreduce_adam(arena.layout["W"], arena.layout["G"], arena.layout["U"], arena.layout["V"], h_off,
+                                     arena.layout["R"], arena.block_group.data_ptr(), lrm, wd, ex, arena.hyper.data_ptr(),
+                                     arena.adam_t.data_ptr(), float(b1), float(b2), float(eps),
+                                     float(inv_k if inv_k is not None else 1.0 / self.size), int(lo), int(hi), int(bool(wire16)), a,
+                                     self._blocks(max_blocks), self._stream(), int(bool(push_master)))
+        return a
+
+    def adam_advance(self, arena):
+        """``arena.adam_t += 1`` on the current stream (one tiny kernel; graph-capturable)."""
+        self.L.adam_advance(arena.adam_t.data_ptr(), self._stream())
+
+    def push_region_slices(self, arena, region, lo, hi, max_blocks=None):
+        """All ranks: push the slice of fp32 region ``region`` ('W', 'U', 'V') each rank owns in the two-shot partition of
+        ``[lo, hi)`` to the peers."""
+        from ..ops.cuda_impl import _table
+        lrm, wd, ex = _table(arena)
+        self.pa.push_region_slices(arena.layout[region], arena.block_group.data_ptr(), lrm, wd, ex, int(lo), int(hi),
+                                   self._blocks(max_blocks), self._stream())
+
     def push_master_slices(self, arena, lo, hi, max_blocks=None):
         """All ranks: push the fp32 master weights of the slice each rank owns in the two-shot partition of ``[lo, hi)`` to the
         peers (re-synchronises ``W`` after fused steps that ran with ``push_master=False``)."""
-        from ..ops.cuda_impl import _table
-        lrm, wd, ex = _table(arena)
-        self.pa.push_master_slices(arena.layout["W"], arena.block_group.data_ptr(), lrm, wd, ex, int(lo), int(hi),
-                                   self._blocks(max_blocks), self._stream())
+        self.push_region_slices(arena, "W", lo, hi, max_blocks)
 
     def configure_gemm_rs(self, arena, ranges):
         """Arm the reduce-scatter epilogue of the GEMM for the given single-tensor buckets ``[(lo, hi), …]`` (element ranges

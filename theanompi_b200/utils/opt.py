@@ -21,6 +21,9 @@ flat arena (one launch each):
 (m = per-group lr multiplier: 1 for 'W', 2 for 'b'; η only on 'W'; BN gamma/beta
 are updated locally in the pre step and never exchanged, ``opt.py:207-226``.)
 
+Models with ``optimizer = 'adam'`` use :func:`_pre_post_adam` instead (send = G, Adam
+on R / k after the exchange, :class:`FlatAdam`).
+
 The B200 fast path does not use the split at all: the fused exchanger kernels
 (``csrc/comm_kernels.cu``) read every peer's G over NVLink, average, and apply
 the momentum/weight-decay/lr update in the same pass — :class:`FlatSGD` is the
@@ -100,37 +103,55 @@ class FlatSGD(object):
 
 
 class FlatAdam(object):
-    """Adam over the whole arena in one native kernel (``csrc/comm_kernels.cu: adam_flat_kernel``): first moment in the arena's
-    U region, second moment in an extra flat buffer, step counter and lr in device memory — the step is CUDA-graph capturable.
-    The reference's Wide-ResNet uses Keras Adam (``keras_model_zoo/wresnet.py:159``)."""
+    """Adam over the arena in one native kernel (``csrc/comm_kernels.cu: adam_flat_kernel``): first moment in the arena's U
+    region, second moment in its V region, step counter (``arena.adam_t``) and lr in device memory — the step is CUDA-graph
+    capturable.  The reference's Wide-ResNet uses Keras Adam (``keras_model_zoo/wresnet.py:159``)."""
 
     def __init__(self, arena, b1=0.9, b2=0.999, eps=1e-8):
+        arena.ensure_adam_state()
         self.arena, self.b1, self.b2, self.eps = arena, b1, b2, eps
-        self.V = torch.zeros_like(arena.W)
-        self.t = torch.zeros(1, dtype=torch.int64, device=arena.W.device)
 
-    def step(self, lr=None):
+    @property
+    def V(self):
+        return self.arena.V
+
+    @property
+    def t(self):
+        return self.arena.adam_t
+
+    def step(self, lr=None, k=1, src="G", only_local=False, only_exchanged=False, advance=True):
+        """Adam on ``src / k`` (``src`` = the G or R region) for all groups, only the non-exchanged (BN) ones or only the
+        exchanged ones; ``advance=False`` leaves the step counter for a later call of the same step."""
         a = self.arena
+        g = getattr(a, src)
         nat = _native_for(a.W)
         if nat is not None:
             from ..ops.cuda_impl import L, _table, _p, _st
             lrm, wd, ex = _table(a)
-            L().adam_flat(a.W.data_ptr(), a.G.data_ptr(), a.U.data_ptr(), self.V.data_ptr(), _p(a.H), a.block_group.data_ptr(), lrm, wd, ex,
-                          a.hyper.data_ptr(), self.t.data_ptr(), float(self.b1), float(self.b2), float(self.eps), 0, int(a.numel), _st(a.W))
+            filt = 1 if only_local else (2 if only_exchanged else 0)
+            L().adam_flat(a.W.data_ptr(), g.data_ptr(), a.U.data_ptr(), a.V.data_ptr(), _p(a.H), a.block_group.data_ptr(), lrm, wd, ex,
+                          a.hyper.data_ptr(), a.adam_t.data_ptr(), float(self.b1), float(self.b2), float(self.eps), 0, int(a.numel),
+                          _st(a.W), inv_k=1.0 / k, filter=filt, advance=int(bool(advance)))
             return
         lr = float(a.hyper[0]) if lr is None else lr
-        self.t += 1
-        t = float(self.t)
-        g = a.G + a.wd_vector() * a.W
-        a.U.mul_(self.b1).add_(g, alpha=1 - self.b1)
-        self.V.mul_(self.b2).addcmul_(g, g, value=1 - self.b2)
-        mh, vh = a.U / (1 - self.b1 ** t), self.V / (1 - self.b2 ** t)
-        a.W.sub_(lr * a.lr_mult_vector() * mh / (vh.sqrt() + self.eps))
+        t = float(int(a.adam_t) + 1)
+        lrm, wd = a.lr_mult_vector(), a.wd_vector()
+        if only_local or only_exchanged:
+            ex = a.exch_vector()
+            idx = (~ex if only_local else ex).nonzero().squeeze(1)
+            if idx.numel():
+                w2, m2, v2 = a.W[idx].clone(), a.U[idx].clone(), a.V[idx].clone()
+                ref.adam_flat(w2, g[idx], m2, v2, lrm[idx], wd[idx], lr, self.b1, self.b2, self.eps, t, 1.0 / k)
+                a.W[idx], a.U[idx], a.V[idx] = w2, m2, v2
+        else:
+            ref.adam_flat(a.W, g, a.U, a.V, lrm, wd, lr, self.b1, self.b2, self.eps, t, 1.0 / k)
+        if advance:
+            a.adam_t += 1
         if a.H is not None:
             a.H.copy_(a.W)
 
     def state_dict(self):
-        return {"V": self.V.detach().cpu(), "t": int(self.t)}
+        return {"V": self.V.detach().cpu().clone(), "t": int(self.t)}
 
     def load_state_dict(self, sd):
         self.V.copy_(sd["V"].to(self.V.device)); self.t.fill_(int(sd["t"]))
@@ -219,6 +240,27 @@ def _pre_post_sgd(model, k):
     return pre, post, "G"
 
 
+def _pre_post_adam(model, k):
+    """Synchronous data-parallel Adam: average the gradients, then one Adam step (= single-process Adam on the global batch).
+    pre : local Adam step of the non-exchanged (BN) groups on the rank's own G            send = G
+    post: Adam step of the exchanged groups on R / k (R = Σ_ranks G), then t += 1
+    The fused strategies compute the same thing inside the exchange kernels."""
+    adam = model.adam
+
+    def pre():
+        if k == 1:
+            adam.step()
+            return
+        adam.step(only_local=True, advance=False)
+
+    def post():
+        if k == 1:
+            return
+        adam.step(k=k, src="R", only_exchanged=True)
+
+    return pre, post, "G"
+
+
 def _publish(model, pre, post, send_region, k):
     a = model.arena
     mask = a.exchanged_mask()
@@ -252,6 +294,8 @@ def _clip_paramlist(param_list, scale=10):
 
 
 def prepare_update_dict(model, k=1, aggregate="momentum"):
+    if getattr(model, "optimizer", "msgd") == "adam":
+        return _publish(model, *_pre_post_adam(model, k), k)
     if model.use_momentum:
         if aggregate == "gradient":
             return _BSP_MSGD(model, model.use_nesterov_momentum, k=k)
